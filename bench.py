@@ -16,6 +16,10 @@ so per-GPU work is fixed: weak scaling.
 Rank 0 prints ONE JSON line.  `value` is device-timed with keys resident in
 HBM; `e2e` goes through the public dpf-API call with pinned HOST keys, H2D and
 D2H inside the timed region.
+
+--dump-outputs DIR saves the answers the last timed step computed (DIR/answers.npy).  Table and
+keys come from fixed seeds, so two builds run with the same arguments can be compared answer for
+answer.
 """
 import argparse
 import json
@@ -39,6 +43,7 @@ BASELINE_PUBLISHED = {  # BASELINE.md section 1 (reference README.md:129-146), V
     ("salsa20", 1 << 14): 145646, ("salsa20", 1 << 16): 54892, ("salsa20", 1 << 18): 16650, ("salsa20", 1 << 20): 3894,
     ("chacha20", 1 << 14): 139590, ("chacha20", 1 << 16): 56120, ("chacha20", 1 << 18): 16086, ("chacha20", 1 << 20): 4054,
 }
+DUMP_MAX_BYTES = 60 << 20     # --dump-outputs: stays under 64 MB with the .npy headers
 
 
 _REAL_STDOUT = None
@@ -78,7 +83,15 @@ def parse_args():
     ap.add_argument("--no-parity", action="store_true", help="skip the post-timing parity check of the timed batch")
     ap.add_argument("--reduce", default="nccl", choices=["nccl", "fused"],
                     help="N>1: NCCL reduce of the partials, or the kernel's peer-memory red.add epilogue")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the [batch, entry] result of the last timed step to DIR/answers.npy (float64, exact "
+                         "for int32; a seeded sample of rows above %d MiB) so two builds can be compared" % (DUMP_MAX_BYTES >> 20))
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 def bytes_per_dpf(n, entry):
@@ -410,11 +423,12 @@ def parity_check(h, d, world, prf, table, keys_a, keys_b, alphas, n_oracle=4):
 
 
 def measure(h, prf_name, n, entry, batch, steps, warmup, world=None, axis="entries", reduce="nccl",
-            e2e=True, parity=4, settle_s=0.0, subtree_log2=0, sampler=None):
+            e2e=True, parity=4, settle_s=0.0, subtree_log2=0, sampler=None, keep_output=False):
     """One configuration: eval_init, warm-up, `steps` device-timed steps (CUDA events on the launching
     stream, max over ranks, L2 flushed before every step), optionally the end-to-end leg through the
     public host-buffer API, and the parity check of the timed batch.  world=1 on a multi-rank run
-    means: this rank alone, no collectives (other ranks must not call)."""
+    means: this rank alone, no collectives (other ranks must not call).  keep_output: res["output"] is
+    a host copy of what the last timed step returned (the complete result on rank 0 only)."""
     import dpf as dpf_mod
     from sharded import ShardedDPF
     torch = h.torch
@@ -439,7 +453,7 @@ def measure(h, prf_name, n, entry, batch, steps, warmup, world=None, axis="entri
     out_dev = torch.empty((batch, entry), dtype=torch.int32, device=h.dev)
 
     def step_device():
-        d.eval_gpu_device(keys_dev, out_dev)
+        return d.eval_gpu_device(keys_dev, out_dev)
 
     nwarm = max(warmup, 3)
     t_warm = time.perf_counter()
@@ -471,11 +485,13 @@ def measure(h, prf_name, n, entry, batch, steps, warmup, world=None, axis="entri
     for k in range(steps):
         h.flush.zero_()                       # cold L2 at the start of every timed step
         starts[k].record()
-        step_device()
+        last = step_device()
         ends[k].record()
     torch.cuda.synchronize()
     h.barrier(world)
     t_wall = time.perf_counter() - t_wall0
+    # copied before anything else runs: the key-split path hands out a buffer that the next call reuses
+    output = last.cpu().numpy().copy() if (keep_output and last is not None) else None
     clocks = sampler.stop() if sampler else None
     dev_ms = h.max_over_ranks(sum(s.elapsed_time(e) for s, e in zip(starts, ends)), world)
     # per-step times (max over ranks, step by step): the median is what the sub-millisecond extras report
@@ -487,7 +503,7 @@ def measure(h, prf_name, n, entry, batch, steps, warmup, world=None, axis="entri
     res = {"value": batch * steps / (dev_ms / 1e3), "ms_per_step": dev_ms / steps, "ms_per_step_median": ms_median,
            "launches_per_step": launches_per_step,
            "warmup_effective": nwarm + extra_n, "wall_s_timed_region": t_wall, "clocks": clocks, "axis": axis_used,
-           "batch": batch, "e2e": None, "parity_check": None}
+           "batch": batch, "e2e": None, "parity_check": None, "output": output}
 
     if e2e:   # end to end through the public API: pinned HOST keys in, HOST result out, every step
         keys_host = torch.from_numpy(keys_a).pin_memory()
@@ -514,6 +530,18 @@ def measure(h, prf_name, n, entry, batch, steps, warmup, world=None, axis="entri
     return res
 
 
+def dump_outputs(dirname, out):
+    """int32 [batch, entry] answers as float64 (every int32 is exact there).  Above DUMP_MAX_BYTES a
+    fixed, seeded sample of rows is kept, in row order, and the rows taken go to answer_rows.npy."""
+    os.makedirs(dirname, exist_ok=True)
+    max_rows = max(1, DUMP_MAX_BYTES // (8 * (out.shape[1] + 1)))
+    if out.shape[0] > max_rows:
+        rows = np.sort(np.random.RandomState(0).choice(out.shape[0], max_rows, replace=False))
+        out = out[rows]
+        np.save(os.path.join(dirname, "answer_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(dirname, "answers.npy"), out.astype(np.float64))
+
+
 def run_ours(args):
     h = Harness(args)
     world, rank = h.world, h.rank
@@ -526,8 +554,11 @@ def run_ours(args):
     axis = args.axis if (args.strong or args.axis != "auto") else "entries"
     m = measure(h, args.prf, n, entry, batch, args.steps, args.warmup, axis=axis, reduce=args.reduce,
                 e2e=not args.no_e2e, parity=0 if args.no_parity else 4, settle_s=0.5,
-                subtree_log2=args.subtree_log2, sampler=sampler)
+                subtree_log2=args.subtree_log2, sampler=sampler, keep_output=bool(args.dump_outputs))
     table = m.pop("table")
+    output = m.pop("output")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, output)
     value, clocks = m["value"], m["clocks"]
 
     # ---- bounded sweep over the other sizes / PRFs the north star names (N = 1), the BASELINE

@@ -1,8 +1,9 @@
-"""The CPU oracle against (a) the golden vectors produced by the real reference and
-(b) the real reference itself when oracle/_ref is built.  No GPU."""
+"""The CPU oracle against the golden vectors produced by the real reference.  No GPU."""
+import os
 import random
 
 import numpy as np
+import pytest
 
 from common import dot_u32, formula_table
 
@@ -87,35 +88,52 @@ def test_dot_range_matches_full(oracle, golden):
     assert np.array_equal((a + b).astype(np.int32)[0], golden["dots_a"][ci])
 
 
-# ---- against the real reference (build container only) --------------------
+# ---- against the real reference's answers (tests/golden/make_reference_checks.py cpu) ----
 
-def test_oracle_matches_reference_prf(oracle, ref):
+@pytest.fixture(scope="module")
+def reference_cpu():
+    return np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_cpu_v1.npz"))
+
+
+def _u128(lo_hi):
+    return int(lo_hi[0]) | (int(lo_hi[1]) << 64)
+
+
+def test_oracle_matches_reference_prf(oracle, reference_cpu):
     r = random.Random(7)
-    for _ in range(200):
+    seeds, outs = reference_cpu["prf_seed"], reference_cpu["prf_out"]
+    assert seeds.shape[0] == 200
+    for si in range(seeds.shape[0]):
         s = r.getrandbits(128)
+        assert s == _u128(seeds[si])
         for prf in range(4):
             for pos in (0, 1):
-                assert oracle.prf(prf, s, pos) == ref.prf(prf, s, pos)
+                assert oracle.prf(prf, s, pos) == _u128(outs[prf, si, pos])
 
 
-def test_oracle_matches_reference_gen_and_eval(oracle, ref):
+def test_oracle_matches_reference_gen_and_eval(oracle, reference_cpu):
     r = random.Random(11)
+    meta = reference_cpu["gen_meta"]
+    full = reference_cpu["eval_full_a"]
+    ci, off = 0, 0
     for prf in range(4):
         for n in (2, 4, 256, 2048):
             for _ in range(3):
                 alpha, seed32 = r.randrange(n), r.getrandbits(32)
+                assert tuple(int(v) for v in meta[ci]) == (prf, n, alpha, seed32)
                 ka, kb = oracle.gen(alpha, n, seed32, prf)
-                ra, rb = ref.gen(alpha, n, seed32, prf)
+                ra, rb = reference_cpu["gen_keys_a"][ci], reference_cpu["gen_keys_b"][ci]
                 assert np.array_equal(ka, ra) and np.array_equal(kb, rb)
-                assert np.array_equal(oracle.eval_full(ka, prf), ref.eval_full(ka, prf))
-                for idx in (0, alpha, n - 1):
-                    assert oracle.eval_flat(kb, idx, prf) == ref.eval_flat(kb, idx, prf)
+                assert np.array_equal(oracle.eval_full(ka, prf), full[off:off + n])
+                for j, idx in enumerate((0, alpha, n - 1)):
+                    assert oracle.eval_flat(kb, idx, prf) == _u128(reference_cpu["eval_flat_b"][ci, j])
+                ci, off = ci + 1, off + n
+    assert ci == meta.shape[0] and off == full.shape[0]
 
 
-def test_reference_baseline_harness(oracle, ref):
+def test_reference_baseline_harness(oracle, reference_cpu):
     """ref_eval_dot_mt (the --impl reference timing leg) computes the same inner product."""
     n = 512
     t = formula_table(n, 16)
     keys = np.stack([oracle.gen(i * 37 % n, n, 50 + i, 2)[0] for i in range(5)])
-    got = ref.eval_dot_mt(keys, 2, t, 0, n, 3)
-    assert np.array_equal(got, oracle.eval_dot(keys, 2, t))
+    assert np.array_equal(reference_cpu["harness_dot"], oracle.eval_dot(keys, 2, t))
