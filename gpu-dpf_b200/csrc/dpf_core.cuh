@@ -481,6 +481,12 @@ template <int PRF, bool FULL, class Env>
 DPF_HD void eval_subtree(Env &env, Seed seed, int s, int level_base)
 {
     int h = s;
+    /* AES: the pending right child of height 1 is taken right after the next leaf pair, so it stays
+     * in registers instead of going through env.push/pop -- one 16-byte store and load fewer on the
+     * shared-memory pipe that binds the AES kernel, per height-2 node.  The selects that cost are
+     * extra issue slots, which is what binds Salsa/ChaCha, so they keep the stack. */
+    constexpr bool REG_SIBLING = (PRF == PRF_AES128);
+    Seed right1 = seed;
     const uint32_t npairs = 1u << (s - 1);
     for (uint32_t i = 0; i < npairs; i++) {
         while (h > 1) {
@@ -489,7 +495,8 @@ DPF_HD void eval_subtree(Env &env, Seed seed, int s, int level_base)
             const uint32_t bank = seed.x & 1u;
             const int level = level_base + h - 1;
             c1 = add128(c1, env.cw(level, bank, 1));
-            env.push(h - 1, c1);
+            if (REG_SIBLING && h == 2) right1 = c1;
+            else env.push(h - 1, c1);
             seed = add128(c0, env.cw(level, bank, 0));
             h--;
         }
@@ -504,7 +511,8 @@ DPF_HD void eval_subtree(Env &env, Seed seed, int s, int level_base)
             env.leaf_pair(2 * i, l0.x + env.cw_lo(bank, 0), l1.x + env.cw_lo(bank, 1));
         }
         h = ctz32(i + 1) + 1;
-        if (h < s) seed = env.pop(h);
+        if (REG_SIBLING && h == 1 && s > 1) seed = right1;
+        else if (h < s) seed = env.pop(h);
     }
 }
 

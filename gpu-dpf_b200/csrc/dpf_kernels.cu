@@ -25,7 +25,9 @@
  *   MAC         = only the low 32 bits of a leaf survive (dpf_wrapper.cu:182),
  *                 so the product is 32-bit IMADs against an int32 table stored
  *                 in breadth-first leaf order (4x less table traffic than the
- *                 reference's 128-bit table, ~20x fewer MAC instructions).
+ *                 reference's 128-bit table, ~20x fewer MAC instructions).  With
+ *                 4+ keys per warp the 4 lanes of a quad split the row into 4
+ *                 column slices and trade their leaves by shuffle (DevEnv, QUAD).
  *   corrections = the 32 keys' correction words live in shared memory, laid out
  *                 [level][bank][bit][key] so a warp's 16-byte reads are
  *                 conflict free.
@@ -44,9 +46,10 @@
  *                 top-phase tickets for the next launch.  (The reference's step is
  *                 cudaMemcpy + kernel + cudaMemcpy with a stream created per call,
  *                 dpf_wrapper.cu:150-176; ours was memset, memset, kernel, kernel.)
- *   wide rows   = NV uint4 of a table row per pass (16/32/64 int32 columns): the
- *                 first 64 bytes of both rows are prefetched before the leaf
- *                 expansion, the rest streamed chunk by chunk during the MAC.
+ *   wide rows   = NV uint4 of a table row per pass (16/32/64 int32 columns), loaded
+ *                 before the leaf expansion: a lane's NV/4 uint4 slice of both rows
+ *                 (quad layout), or the first 64 bytes of both rows with the rest
+ *                 streamed chunk by chunk during the MAC (1 or 2 keys per warp).
  *   scheduling  = persistent blocks; warps draw subtrees from a per-key-group
  *                 ticket counter (atomicAdd), blocks migrate to the next key
  *                 group when theirs runs dry, partial sums leave through
@@ -124,8 +127,21 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void *src, uint32_t
 }  // namespace tma
 
 /* ---- per-thread environment for the shared traversal code ---------------- */
-template <int PRF, int NV, int THREADS, int MODE>
+/*
+ * Two layouts of the inner product (MAC):
+ *   QUAD = false  every lane multiplies its own key's leaves against the whole row: it loads
+ *                 all NV uint4 of both rows of a leaf pair (the per-lane layout; the only one
+ *                 possible with 1 or 2 keys per warp, where no two lanes share a subtree);
+ *   QUAD = true   (keys per warp >= 4) the 4 lanes of a quad hold 4 keys of the same subtree,
+ *                 and quad lane j owns the column slice {uint4 j, j+4, j+8, ...}: it loads
+ *                 NV/4 uint4 of each row, takes its partners' leaves with 6 shuffles, and
+ *                 accumulates 4 keys x its columns.  Same IMAD count, 4x fewer row bytes
+ *                 through the LSU per leaf pair (a broadcast LDG.128 still costs 4 wavefronts).
+ *                 acc[16*c + 4*m + e] is key (kslot ^ m), column 4*(4c + j) + e.
+ */
+template <int PRF, int NV, int THREADS, int MODE, bool QUAD>
 struct DevEnv {
+    static constexpr int ROW_V = QUAD ? NV / 4 : 4;   /* uint4 of each row held in registers */
     typename TablePolicy<PRF>::type ta;
     const uint4 *cw_lane;       /* &cw_s[lane]; entry (level,bank,bit) at +((level*2+bank)*2+bit)*32 */
     const uint32_t *cwlo_lane;  /* &cwlo_s[lane]; entry (bank,bit) at +(bank*2+bit)*32 */
@@ -133,8 +149,10 @@ struct DevEnv {
     int stack_split;
     const uint4 *rows;          /* first row of the current subtree, at this pass's column */
     uint32_t row_stride_v;
+    uint32_t qlane;             /* QUAD: lane & 3, the column slice this lane owns */
     uint32_t acc[4 * NV];
-    uint4 ra[4], rb[4];         /* prefetched first 64 bytes of the two rows of a leaf pair */
+    uint4 ra[ROW_V], rb[ROW_V]; /* prefetched row data of a leaf pair: QUAD, this lane's slice of both
+                                 * rows; otherwise the first 64 bytes of both */
     uint32_t *leaf_out;         /* leaf cache slot of the subtree's first leaf for this lane, or null */
     uint4 *front_out;           /* MODE_FRONTIER: &frontier[(kg*nfront + first node)*kpw + key slot] */
     uint32_t kpw;               /* keys per warp */
@@ -178,52 +196,87 @@ struct DevEnv {
 
     __device__ __forceinline__ void leaf_prefetch(uint32_t local_pos)
     {
-        if (STAGED) {
+        if constexpr (STAGED) {
             if (tile_pending) {
                 tma::mbar_wait(tile_bar, tile_phase);
                 tile_phase ^= 1u;
                 tile_pending = false;
             }
-            const uint4 *r = tile + (size_t)local_pos * 4;
+            const uint4 *r = tile + (size_t)local_pos * 4;   /* 64-byte rows: NV = 4 */
+            if constexpr (QUAD) {
+                ra[0] = r[qlane];
+                rb[0] = r[4 + qlane];
+            } else {
 #pragma unroll
-            for (int j = 0; j < 4; j++) ra[j] = r[j];
+                for (int j = 0; j < 4; j++) ra[j] = r[j];
 #pragma unroll
-            for (int j = 0; j < 4; j++) rb[j] = r[4 + j];
-        } else if (MAC) {
-            const uint4 *r = rows + (size_t)local_pos * row_stride_v;
+                for (int j = 0; j < 4; j++) rb[j] = r[4 + j];
+            }
+        } else if constexpr (MAC) {
+            if constexpr (QUAD) {
+                const uint4 *r = rows + (size_t)local_pos * row_stride_v + qlane;
 #pragma unroll
-            for (int j = 0; j < 4; j++) ra[j] = __ldg(r + j);
+                for (int c = 0; c < ROW_V; c++) ra[c] = __ldg(r + 4 * c);
 #pragma unroll
-            for (int j = 0; j < 4; j++) rb[j] = __ldg(r + row_stride_v + j);
+                for (int c = 0; c < ROW_V; c++) rb[c] = __ldg(r + row_stride_v + 4 * c);
+            } else {
+                const uint4 *r = rows + (size_t)local_pos * row_stride_v;
+#pragma unroll
+                for (int j = 0; j < 4; j++) ra[j] = __ldg(r + j);
+#pragma unroll
+                for (int j = 0; j < 4; j++) rb[j] = __ldg(r + row_stride_v + j);
+            }
         }
     }
     __device__ __forceinline__ void leaf_pair(uint32_t local_pos, uint32_t v0, uint32_t v1)
     {
-        if (MAC) {
+        if constexpr (MAC) {
             if (leaf_out != nullptr) {   /* coalesced: 32 keys x 4 bytes per leaf */
                 leaf_out[(size_t)local_pos * 32] = v0;
                 leaf_out[(size_t)(local_pos + 1) * 32] = v1;
             }
-            const uint4 *r = rows + (size_t)local_pos * row_stride_v;
+            if constexpr (QUAD) {
+                /* slot m: the leaves of key kslot ^ m, held by quad lane qlane ^ m */
+                uint32_t w0[4], w1[4];
+                w0[0] = v0;
+                w1[0] = v1;
 #pragma unroll
-            for (int c = 0; c < NV / 4; c++) {
-                uint4 na[4], nb[4];
-                if (c + 1 < NV / 4) {   /* next 64 bytes of both rows while this chunk is multiplied */
-#pragma unroll
-                    for (int j = 0; j < 4; j++) na[j] = __ldg(r + 4 * (c + 1) + j);
-#pragma unroll
-                    for (int j = 0; j < 4; j++) nb[j] = __ldg(r + row_stride_v + 4 * (c + 1) + j);
+                for (int m = 1; m < 4; m++) {
+                    w0[m] = __shfl_xor_sync(0xffffffffu, v0, m);
+                    w1[m] = __shfl_xor_sync(0xffffffffu, v1, m);
                 }
 #pragma unroll
-                for (int j = 0; j < 4; j++) {
-                    acc[16 * c + 4 * j + 0] += v0 * ra[j].x + v1 * rb[j].x;
-                    acc[16 * c + 4 * j + 1] += v0 * ra[j].y + v1 * rb[j].y;
-                    acc[16 * c + 4 * j + 2] += v0 * ra[j].z + v1 * rb[j].z;
-                    acc[16 * c + 4 * j + 3] += v0 * ra[j].w + v1 * rb[j].w;
-                }
-                if (c + 1 < NV / 4) {
+                for (int c = 0; c < ROW_V; c++) {
 #pragma unroll
-                    for (int j = 0; j < 4; j++) { ra[j] = na[j]; rb[j] = nb[j]; }
+                    for (int m = 0; m < 4; m++) {
+                        acc[16 * c + 4 * m + 0] += w0[m] * ra[c].x + w1[m] * rb[c].x;
+                        acc[16 * c + 4 * m + 1] += w0[m] * ra[c].y + w1[m] * rb[c].y;
+                        acc[16 * c + 4 * m + 2] += w0[m] * ra[c].z + w1[m] * rb[c].z;
+                        acc[16 * c + 4 * m + 3] += w0[m] * ra[c].w + w1[m] * rb[c].w;
+                    }
+                }
+            } else {
+                const uint4 *r = rows + (size_t)local_pos * row_stride_v;
+#pragma unroll
+                for (int c = 0; c < NV / 4; c++) {
+                    uint4 na[4], nb[4];
+                    if (c + 1 < NV / 4) {   /* next 64 bytes of both rows while this chunk is multiplied */
+#pragma unroll
+                        for (int j = 0; j < 4; j++) na[j] = __ldg(r + 4 * (c + 1) + j);
+#pragma unroll
+                        for (int j = 0; j < 4; j++) nb[j] = __ldg(r + row_stride_v + 4 * (c + 1) + j);
+                    }
+#pragma unroll
+                    for (int j = 0; j < 4; j++) {
+                        acc[16 * c + 4 * j + 0] += v0 * ra[j].x + v1 * rb[j].x;
+                        acc[16 * c + 4 * j + 1] += v0 * ra[j].y + v1 * rb[j].y;
+                        acc[16 * c + 4 * j + 2] += v0 * ra[j].z + v1 * rb[j].z;
+                        acc[16 * c + 4 * j + 3] += v0 * ra[j].w + v1 * rb[j].w;
+                    }
+                    if (c + 1 < NV / 4) {
+#pragma unroll
+                        for (int j = 0; j < 4; j++) { ra[j] = na[j]; rb[j] = nb[j]; }
+                    }
                 }
             }
         } else if (MODE == MODE_EXPAND && key_valid) {
@@ -283,8 +336,9 @@ __device__ __forceinline__ unsigned long long global_ns()
     return t;
 }
 
-/* `quota`: tickets this WARP may draw in this call over all key groups (0xffffffff = no limit). */
-template <int PRF, int NV, int THREADS, int MODE>
+/* `quota`: tickets this WARP may draw in this call over all key groups (0xffffffff = no limit).
+ * QUAD: the MAC layout of DevEnv; needs at least 4 keys per warp. */
+template <int PRF, int NV, int THREADS, int MODE, bool QUAD = false>
 __device__ __forceinline__ void run_phase(const EvalParams &p, const PhaseParams &ph,
                                           const typename TablePolicy<PRF>::type &ta, uint32_t quota = 0xffffffffu)
 {
@@ -303,8 +357,9 @@ __device__ __forceinline__ void run_phase(const EvalParams &p, const PhaseParams
     const uint32_t sslot = (uint32_t)lane >> p.kpw_log2;
     const uint32_t ntickets = ph.nsub >> spw_log2;
 
-    DevEnv<PRF, NV, THREADS, MODE> env;
+    DevEnv<PRF, NV, THREADS, MODE, QUAD> env;
     env.ta = ta;
+    env.qlane = (uint32_t)lane & 3u;
     env.cw_lane = cw_s + kslot;
     env.cwlo_lane = cwlo_s + kslot;
     env.kpw = (uint32_t)kpw;
@@ -457,7 +512,23 @@ __device__ __forceinline__ void run_phase(const EvalParams &p, const PhaseParams
 #pragma unroll
                 for (int e = 0; e < 4 * NV; e++) env.acc[e] += __shfl_xor_sync(0xffffffffu, env.acc[e], off);
             }
-            if (env.key_valid && sslot == 0) {
+            if (QUAD && sslot == 0) {
+                /* 4 keys x this lane's column slice; a lane past the group's last key computed that
+                 * key's leaves again (clamped correction words), so every key has its own mask */
+#pragma unroll
+                for (int m = 0; m < 4; m++) {
+                    const int key_m = g_key_first + (kslot ^ m);
+                    if (key_m > g_key_last) continue;
+                    uint32_t *o = p.out + (size_t)key_m * p.out_stride + p.col_off;
+#pragma unroll
+                    for (int c = 0; c < NV / 4; c++)
+#pragma unroll
+                        for (int e = 0; e < 4; e++) {
+                            const uint32_t col = 4u * (4u * c + env.qlane) + e;
+                            if (col < p.ncols) atomicAdd(o + col, env.acc[16 * c + 4 * m + e]);
+                        }
+                }
+            } else if (!QUAD && env.key_valid && sslot == 0) {
                 uint32_t *o = p.out + (size_t)key * p.out_stride + p.col_off;
 #pragma unroll
                 for (int e = 0; e < 4 * NV; e++)
@@ -525,7 +596,16 @@ dpf_eval_kernel(const __grid_constant__ EvalParams p)
                 for (uint32_t i = tid; i < p.rearm_words; i += THREADS) p.rearm[i] = 0u;
         }
     }
-    run_phase<PRF, NV, THREADS, MODE>(p, p.main, ta);
+    /* ChaCha measured 0.5-1.2 % slower with the quad MAC layout on a B200 (n = 2^16 and 2^20,
+     * B = 512; AES +3.5 %, Salsa +0.4 %), so it keeps the per-lane layout */
+    constexpr bool QUAD_MAC = PRF != PRF_CHACHA20;
+    if constexpr (QUAD_MAC && (MODE == MODE_FUSED || MODE == MODE_GROUPED || MODE == MODE_FUSED_TMA)) {
+        /* kpw_log2 is the same for the whole launch: one of the two MAC layouts runs */
+        if (p.kpw_log2 >= 2) run_phase<PRF, NV, THREADS, MODE, true>(p, p.main, ta);
+        else run_phase<PRF, NV, THREADS, MODE, false>(p, p.main, ta);
+    } else {
+        run_phase<PRF, NV, THREADS, MODE>(p, p.main, ta);
+    }
     if (stamp) stamp[4] = global_ns();
 }
 
